@@ -19,6 +19,7 @@ runs on the GPU as `c1` and is checked against tests/golden/path1_c1.json.  BM25
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            our CUDA path
   python bench.py --impl reference ...                          the reference's CPU path (oracle port)
+  python bench.py --dump-outputs DIR ...                        also write the last timed step's result as DIR/*.npy
 """
 import argparse
 import hashlib
@@ -144,6 +145,27 @@ def registers_checksum(regs, owned=None):
 
 def _i64(x):
     return x - (1 << 64) if x >= (1 << 63) else x
+
+
+DUMP_MAX_ENTRIES = 1 << 20   # 40 bytes per result entry (f64 centrality + 4 x f64 id words): 40 MB at most
+DUMP_SEED = 20240917
+
+
+def dump_outputs(out_dir, ids_lo, ids_hi, values, stats):
+    """--dump-outputs: what one HarmonicCentrality step hands its caller, as .npy files that two builds can be compared on.
+    centrality.npy (f64) and node_ids.npy (f64, the u128 id as four exact 32-bit words, low word first) hold the result
+    entries, or a fixed seeded sample of DUMP_MAX_ENTRIES of them (same positions for the same result length);
+    n_changed.npy (f64) holds the changed-node count of every iteration."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    k = len(values)
+    idx = np.arange(k)
+    if k > DUMP_MAX_ENTRIES:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(k, DUMP_MAX_ENTRIES, replace=False))
+    words = np.stack([np.asarray(ids_lo)[idx], np.asarray(ids_hi)[idx]], axis=1).astype(np.uint64).view(np.uint32)
+    np.save(os.path.join(out_dir, "centrality.npy"), np.asarray(values, np.float64)[idx])
+    np.save(os.path.join(out_dir, "node_ids.npy"), words.astype(np.float64))
+    np.save(os.path.join(out_dir, "n_changed.npy"), np.array([s["n_changed"] for s in stats], np.float64))
 
 
 def host_threads():
@@ -355,12 +377,15 @@ def main():
                     "list, NVSwitch multicast) on one staged graph in one process and print one JSON line; no bench line")
     ap.add_argument("--ref-budget-s", type=float, default=170.0, help="--impl reference: wall budget of the timed loops")
     ap.add_argument("--write-golden", action="store_true", help="N=1, after a green oracle check: rewrite tests/golden/path1_c2.json")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="N=1: write the last timed step's result (sampled to <= 40 MB) as DIR/*.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 0)
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and (world > 1 or args.impl != "ours"):
+        ap.error("--dump-outputs is supported for the 1-GPU CUDA path only")
 
     if args.impl == "reference":
         if rank == 0:
@@ -429,6 +454,8 @@ def main():
         ms_total = ev0.elapsed_time(ev1)
         prof = dg.profile()
         dg.set_profiling(False)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, *dg.result(), stats_last)
         value = E * tot_iters / (ms_total * 1e-3)
         iters = tot_iters // args.steps
         cap = {}
