@@ -56,7 +56,22 @@ SB200_API void sb200_segment_destroy(sb200_segment* seg);
 SB200_API int sb200_term_info_store_decode(const uint8_t* store, uint64_t len, int device, sb200_term_info* infos, uint64_t cap,
                                            uint64_t* n_terms);
 
+/* The positions half of the same store: positions_range [start, end) of every term, the end being the next term's start
+ * (term_info_store.rs:66-91), min(cap, n) entries; what sb200_segment_attach_positions takes. */
+SB200_API int sb200_term_info_store_decode_positions(const uint8_t* store, uint64_t len, int device, uint64_t* pos_start, uint64_t* pos_end,
+                                                     uint64_t cap, uint64_t* n_terms);
+
 typedef struct { uint64_t n_terms, n_blocks, n_postings, hbm_bytes; uint32_t max_doc; uint32_t _pad; double stage_ms; } sb200_segment_info;
+
+/* Attaches the field's positions file (tantivy/src/positions/mod.rs:7-30: per term VInt(#blocks), one bit width per block,
+ * 128-delta BitPacker4x blocks, a vint tail of the remaining deltas) to a WithFreqsAndPositions segment (record option 2,
+ * else SB200_EINVAL); term t's bytes are [pos_start[t], pos_end[t]).  The file goes to HBM with a per-128-position block
+ * directory, a 16-byte aligned copy of the bitpacked blocks and, per posting block, the index of its first position (the
+ * skip entries' tf sums, what SkipReader::position_offset accumulates, tantivy/src/postings/skip.rs:244-266).  Every term is
+ * validated first (range inside the file, block count == its term frequency sum / 128, widths <= 32, blocks inside the range,
+ * exactly sum % 128 tail vints): SB200_EFORMAT and nothing attached otherwise.  sb200_segment_get_info().hbm_bytes counts it. */
+SB200_API int sb200_segment_attach_positions(sb200_segment* seg, const uint8_t* positions_file, uint64_t len, const uint64_t* pos_start,
+                                             const uint64_t* pos_end);
 SB200_API int sb200_segment_get_info(const sb200_segment* seg, sb200_segment_info* info);
 
 /* Row-major table of per-document numeric signal scores in HBM ([max_doc][n_cols] f64): what the numeric
@@ -197,6 +212,28 @@ typedef struct {
 SB200_API int sb200_multi_signal_topk_batch(const sb200_multi_signal_batch* batch, uint32_t* docs, double* totals, uint32_t* n_out,
                                             sb200_bm25_stats* stats);
 
+/* Phrase queries with slop 0: tantivy PhraseQuery::new / new_with_offset (query/phrase_query/phrase_query.rs:35-53) collected by
+ * TopDocs on one segment.  Per query the phrase terms term_ords[q][0..lens[q]) with their offsets (any order: the phrase
+ * count does not depend on it); a document matches when every term occurs at (start + offset), PhraseScorer's count is the
+ * number of such starts (phrase_scorer.rs:435-505 with slop 0) and the score is weights[q] * (count / (count +
+ * tf_cache256[fieldnorm id])) (PhraseScorer::score, phrase_scorer.rs:540-549; Bm25Weight::score, bm25.rs:182-196).
+ * weights[q] = Bm25Weight::for_terms(..).weight: (1 + K1) times the f32 idf sum over the terms in offset order
+ * (bm25.rs:98-134), times the boost.  A query with an SB200_NO_TERM among its terms matches nothing (PhraseWeight::phrase_scorer
+ * returns None, phrase_weight.rs:53-62); lens[q] < 2 (phrase_query.rs:49-52) or a segment without positions
+ * (phrase_query.rs:106-118) is SB200_EINVAL.  Outputs as sb200_bm25_topk_batch; stats: postings_scored = sum of the phrase
+ * terms' doc_freq, docs_scored = documents containing every term (the ones whose positions were matched). */
+typedef struct {
+  uint32_t n_queries, n_terms;   /* n_terms = row width, 2 <= n_terms <= SB200_MAX_QUERY_TERMS */
+  const uint32_t* term_ords;     /* [n_queries*n_terms]; SB200_NO_TERM = term absent from this segment */
+  const uint32_t* offsets;       /* [n_queries*n_terms]: PhraseQuery::new_with_offset positions */
+  const uint8_t* lens;           /* [n_queries]: phrase length, 2..n_terms */
+  const float* weights;          /* [n_queries] */
+  const float* tf_cache256;      /* [256] */
+  uint32_t k;
+} sb200_phrase_batch;
+SB200_API int sb200_phrase_topk_batch(sb200_segment* seg, const sb200_phrase_batch* batch, uint32_t* docs, float* scores,
+                                      uint32_t* n_out, sb200_bm25_stats* stats);
+
 /* Host-side writer of tantivy-format posting lists (PostingsSerializer for IndexRecordOption::WithFreqs,
  * tantivy/src/postings/serializer.rs:343-462), used to build synthetic / test segments.  Terms are given
  * CSR-style: term t owns docs[term_off[t]..term_off[t+1]) (ascending) and the matching tfs (>= 1).
@@ -210,6 +247,13 @@ SB200_API int sb200_postings_encode(const uint32_t* docs, const uint32_t* tfs, c
 SB200_API int sb200_postings_encode_ex(const uint32_t* docs, const uint32_t* tfs, const uint64_t* term_off, uint32_t n_terms,
                                        const uint8_t* fieldnorm_ids, uint32_t max_doc, float avg_fieldnorm, int record_option,
                                        uint8_t* out, uint64_t out_cap, uint64_t* out_len, sb200_term_info* infos, int threads);
+/* Host-side writer of the positions file (PositionSerializer, tantivy/src/positions/serializer.rs) for the same CSR: `positions`
+ * holds sum(tfs) entries, every posting's absolute positions (strictly ascending within the document), posting after posting;
+ * a document's deltas restart from 0 (postings/serializer.rs:191-205).  Term t's bytes go to [pos_start[t], pos_end[t])
+ * (both nullable).  Call with out == NULL to get the byte size. */
+SB200_API int sb200_positions_encode(const uint32_t* docs, const uint32_t* tfs, const uint64_t* term_off, uint32_t n_terms,
+                                     const uint32_t* positions, uint8_t* out, uint64_t out_cap, uint64_t* out_len, uint64_t* pos_start,
+                                     uint64_t* pos_end, int threads);
 /* idf(doc_freq, doc_count) = ln(1 + (N - n + 0.5) / (n + 0.5)) in f32 (tantivy/src/query/bm25.rs:52-56,
  * core/src/ranking/bm25.rs:23-27) for an array of doc_freqs; tantivy_weight != 0 returns Bm25Weight.weight = idf * (1 + K1). */
 SB200_API int sb200_bm25_idf(const uint32_t* doc_freq, uint64_t n, uint64_t doc_count, int tantivy_weight, float* out);

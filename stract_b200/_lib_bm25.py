@@ -46,6 +46,11 @@ class MultiSignalBatch(C.Structure):
                 ("slot_boost", C.c_void_p)]
 
 
+class PhraseBatch(C.Structure):
+    _fields_ = [("n_queries", C.c_uint32), ("n_terms", C.c_uint32), ("term_ords", C.c_void_p), ("offsets", C.c_void_p),
+                ("lens", C.c_void_p), ("weights", C.c_void_p), ("tf_cache256", C.c_void_p), ("k", C.c_uint32)]
+
+
 def proto(L, f):
     vp, u32, u64, i32 = C.c_void_p, C.c_uint32, C.c_uint64, C.c_int
     f("sb200_segment_create", i32, vp, u64, vp, u32, vp, u32, i32, i32, C.POINTER(vp))
@@ -65,3 +70,7 @@ def proto(L, f):
     f("sb200_bm25_idf", i32, vp, u64, u64, i32, vp)
     f("sb200_fieldnorm_id_to_value", u32, C.c_uint8)
     f("sb200_fieldnorm_value_to_id", C.c_uint8, u32)
+    f("sb200_term_info_store_decode_positions", i32, vp, u64, i32, vp, vp, u64, C.POINTER(u64))
+    f("sb200_segment_attach_positions", i32, vp, vp, u64, vp, vp)
+    f("sb200_phrase_topk_batch", i32, vp, C.POINTER(PhraseBatch), vp, vp, vp, C.POINTER(Bm25Stats))
+    f("sb200_positions_encode", i32, vp, vp, vp, u32, vp, vp, u64, C.POINTER(u64), vp, vp, i32)

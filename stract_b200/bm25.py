@@ -2,11 +2,12 @@
 
 Mirrors (same names / argument meaning):
   fieldnorm_to_id / id_to_fieldnorm       tantivy/src/fieldnorm/code.rs:1-11
-  Bm25Weight.for_one_term / idf            tantivy/src/query/bm25.rs:52-176      (f32 arithmetic, host side)
+  Bm25Weight.for_one_term / for_terms / idf  tantivy/src/query/bm25.rs:52-176   (f32 arithmetic, host side)
   StractBm25Weight                          core/src/ranking/bm25.rs:23-151
   PostingsWriter                            tantivy/src/postings/serializer.rs (WithFreqs) -- builds segments
   SegmentReader.open                        InvertedIndexReader + FieldNormReader of one field
   TopDocs.with_limit(k) + BooleanQuery      tantivy/src/collector/top_score_collector.rs:360-414
+  PhraseQuery (slop 0) + TopDocs            tantivy/src/query/phrase_query/*.rs, positions/*.rs
   SignalComputer (one text field + numeric signals)   core/src/ranking/computer/mod.rs, initial.rs:79-93
 
 The weights are computed on the host exactly like the reference does before it opens any posting list
@@ -94,6 +95,18 @@ class Bm25Weight:
     def for_one_term(cls, term_doc_freq, total_num_docs, avg_fieldnorm):
         return cls(idf(term_doc_freq, total_num_docs), avg_fieldnorm)
 
+    @classmethod
+    def for_terms(cls, doc_freqs, total_num_docs, avg_fieldnorm):
+        """Bm25Weight::for_terms (bm25.rs:98-134): one term -> for_one_term; several -> the f32 sum of their idfs in the order
+        given (a phrase's terms in offset order), so for three or more terms the order changes the bits."""
+        doc_freqs = [int(d) for d in doc_freqs]
+        if len(doc_freqs) == 1:
+            return cls.for_one_term(doc_freqs[0], total_num_docs, avg_fieldnorm)
+        acc = np.float32(0.0)
+        for d in doc_freqs:
+            acc = np.float32(acc + idf(d, total_num_docs))
+        return cls(acc, avg_fieldnorm)
+
     def score(self, fieldnorm_id, term_freq):
         tf = np.float32(term_freq)
         return np.float32(self.weight * (tf / (tf + self.cache[fieldnorm_id])))
@@ -144,22 +157,51 @@ def encode_postings_csr(docs, tfs, off, fieldnorm_ids, avg_fieldnorm, threads=8,
     return out[:ln.value], infos
 
 
-def decode_term_info_store(store, device=0):
+def encode_positions(term_docs, term_tfs, term_positions, threads=8):
+    """PositionSerializer for a list of terms: term_positions[t] holds the absolute positions of every posting of term t,
+    posting after posting (sum(tfs) entries).  Returns (bytes u8[], pos_start u64[], pos_end u64[])."""
+    n = len(term_docs)
+    off = np.zeros(n + 1, np.uint64)
+    for i, d in enumerate(term_docs):
+        off[i + 1] = off[i] + len(d)
+    cat = lambda xs: np.concatenate([np.asarray(x, np.uint32) for x in xs]) if n else np.zeros(0, np.uint32)  # noqa: E731
+    return encode_positions_csr(cat(term_docs), cat(term_tfs), off, cat(term_positions), threads)
+
+
+def encode_positions_csr(docs, tfs, off, positions, threads=8):
+    L = lib()
+    docs = np.ascontiguousarray(docs, np.uint32); tfs = np.ascontiguousarray(tfs, np.uint32)
+    off = np.ascontiguousarray(off, np.uint64); positions = np.ascontiguousarray(positions, np.uint32)
+    n = off.size - 1
+    ln = C.c_uint64(0)
+    check(L.sb200_positions_encode(_p(docs), _p(tfs), _p(off), n, _p(positions), None, 0, C.byref(ln), None, None, threads))
+    out = np.zeros(max(ln.value, 1), np.uint8)
+    ps = np.zeros(max(n, 1), np.uint64); pe = np.zeros(max(n, 1), np.uint64)
+    check(L.sb200_positions_encode(_p(docs), _p(tfs), _p(off), n, _p(positions), _p(out), out.size, C.byref(ln), _p(ps), _p(pe), threads))
+    return out[:ln.value], ps[:n], pe[:n]
+
+
+def decode_term_info_store(store, device=0, with_positions=False):
     """TermInfoStore bytes (the `.term` store behind tantivy's FST term dictionary) -> TermInfo array, decoded on the
-    device (sb200_term_info_store_decode); pass the result to SegmentReader."""
+    device (sb200_term_info_store_decode); pass the result to SegmentReader.  with_positions=True also returns every
+    term's positions range (pos_start, pos_end), what SegmentReader's `positions` takes."""
     L = lib()
     store = np.ascontiguousarray(store, np.uint8)
     n = C.c_uint64(0)
     check(L.sb200_term_info_store_decode(_p(store), store.size, device, None, 0, C.byref(n)))
     infos = (B.TermInfo * max(n.value, 1))()
     check(L.sb200_term_info_store_decode(_p(store), store.size, device, infos, n.value, C.byref(n)))
-    return infos, int(n.value)
+    if not with_positions:
+        return infos, int(n.value)
+    ps = np.zeros(max(n.value, 1), np.uint64); pe = np.zeros(max(n.value, 1), np.uint64)
+    check(L.sb200_term_info_store_decode_positions(_p(store), store.size, device, _p(ps), _p(pe), n.value, C.byref(n)))
+    return infos, int(n.value), (ps[:n.value], pe[:n.value])
 
 
 class SegmentReader:
     """One field of one segment resident in HBM (postings file + fieldnorms + block directory)."""
 
-    def __init__(self, postings, term_infos, fieldnorm_ids, device=0, record_option=1, total_num_tokens=None):
+    def __init__(self, postings, term_infos, fieldnorm_ids, device=0, record_option=1, total_num_tokens=None, positions=None):
         self._L = lib()
         self._h = C.c_void_p()
         postings = np.ascontiguousarray(postings, np.uint8)
@@ -191,6 +233,17 @@ class SegmentReader:
         # average_fieldnorm = total_num_tokens as f32 / total_num_docs as f32 (bm25.rs:112-114)
         self.average_fieldnorm = np.float32(np.float32(total_num_tokens) / np.float32(max(self.max_doc, 1)))
         self.device = device
+        if positions is not None:
+            self.attach_positions(*positions)
+
+    def attach_positions(self, data, pos_start, pos_end):
+        """The field's positions file and every term's byte range in it (sb200_segment_attach_positions); needs
+        record_option=2 (WithFreqsAndPositions)."""
+        data = np.ascontiguousarray(data, np.uint8)
+        ps = np.ascontiguousarray(pos_start, np.uint64); pe = np.ascontiguousarray(pos_end, np.uint64)
+        if ps.size != self.n_terms or pe.size != self.n_terms:
+            raise ValueError(f"{self.n_terms} terms, {ps.size} / {pe.size} positions ranges")
+        check(self._L.sb200_segment_attach_positions(self._h, _p(data), data.size, _p(ps), _p(pe)))
 
     def info(self):
         si = B.SegmentInfo()
@@ -346,12 +399,62 @@ class TopDocs:
             return docs, scores, n_out, {k_: getattr(st, k_) for k_, _ in B.Bm25Stats._fields_ if not k_.startswith("_")}
         return docs, scores, n_out
 
+    def search_phrase_batch(self, segment, queries, weights=None, average_fieldnorm=None, return_stats=False):
+        """A list of PhraseQuery on one segment (sb200_phrase_topk_batch).  Returns (docs [nq,k], scores [nq,k], n_out [nq]).
+        `weights` ([nq] Bm25Weight.for_terms(..).weight) / `average_fieldnorm` override the segment's own statistics."""
+        nq = len(queries)
+        ords, offs, lens = _phrase_arrays(queries)
+        if weights is None:
+            weights = [Bm25Weight.for_terms([int(segment.doc_freq[t]) if t != NO_TERM else 0 for t in p.term_ords], segment.max_doc,
+                                            segment.average_fieldnorm).weight for p in queries]
+        w = np.zeros(max(nq, 1), np.float32); w[:nq] = np.asarray(weights, np.float32)
+        cache = compute_tf_cache(segment.average_fieldnorm if average_fieldnorm is None else average_fieldnorm)
+        k = self.limit + self.offset
+        docs = host_out((max(nq, 1), k), np.uint32); scores = host_out((max(nq, 1), k), np.float32); n_out = np.zeros(max(nq, 1), np.uint32)
+        b = B.PhraseBatch(nq, ords.shape[1], _p(ords), _p(offs), _p(lens), _p(w), _p(cache), k)
+        st = B.Bm25Stats()
+        check(segment._L.sb200_phrase_topk_batch(segment._h, C.byref(b), _p(docs), _p(scores), _p(n_out), C.byref(st)))
+        docs, scores, n_out = docs[:nq], scores[:nq], n_out[:nq]
+        if self.offset:
+            o = self.offset
+            docs = np.ascontiguousarray(docs[:, o:]); scores = np.ascontiguousarray(scores[:, o:])
+            n_out = (np.maximum(n_out.astype(np.int64) - o, 0)).astype(np.uint32)
+        if return_stats:
+            return docs, scores, n_out, {k_: getattr(st, k_) for k_, _ in B.Bm25Stats._fields_ if not k_.startswith("_")}
+        return docs, scores, n_out
+
     def search(self, segment, term_ords, mode=MODE_AND, weights=None):
         """One query -> list of (score, doc) like the Fruit Vec<(Score, DocAddress)>."""
         t = np.asarray(term_ords, np.uint32)[None, :]
         w = None if weights is None else np.asarray(weights, np.float32)[None, :]
         d, s, n = self.search_batch(segment, t, mode, w)
         return [(float(s[0, i]), int(d[0, i])) for i in range(int(n[0]))]
+
+
+class PhraseQuery:
+    """PhraseQuery::new(terms) / new_with_offset(terms_with_offset) (phrase_query.rs:35-53) with slop 0, terms as ordinals of
+    one field (NO_TERM: absent from the segment).  The terms are kept sorted by offset (stable), as the reference keeps them."""
+
+    def __init__(self, term_ords, offsets=None):
+        term_ords = [int(t) for t in term_ords]
+        offsets = list(range(len(term_ords))) if offsets is None else [int(o) for o in offsets]
+        if len(term_ords) < 2:
+            raise ValueError("A phrase query is required to have strictly more than one term.")
+        if len(offsets) != len(term_ords):
+            raise ValueError("one offset per term")
+        pairs = sorted(zip(offsets, term_ords), key=lambda p: p[0])
+        self.offsets = [o for o, _ in pairs]
+        self.term_ords = [t for _, t in pairs]
+
+
+def _phrase_arrays(queries):
+    nq = len(queries)
+    nt = max([2] + [len(p.term_ords) for p in queries])
+    ords = np.full((max(nq, 1), nt), NO_TERM, np.uint32); offs = np.zeros((max(nq, 1), nt), np.uint32)
+    lens = np.zeros(max(nq, 1), np.uint8)
+    for q, p in enumerate(queries):
+        ords[q, :len(p.term_ords)] = p.term_ords; offs[q, :len(p.offsets)] = p.offsets; lens[q] = len(p.term_ords)
+    return ords, offs, lens
 
 
 class Searcher:
@@ -395,6 +498,36 @@ class Searcher:
                 dead = ((o == NO_TERM) & real).any(axis=1)
                 o[dead] = NO_TERM
             d, sc, n = inner.search_batch(seg, o, mode, weights=weights, average_fieldnorm=self.average_fieldnorm)
+            parts.append((s_ord, d, sc, n))
+        k = top_docs.limit
+        out_seg = np.zeros((nq, k), np.uint32); out_doc = np.zeros((nq, k), np.uint32)
+        out_sc = np.zeros((nq, k), np.float32); out_n = np.zeros(nq, np.uint32)
+        for q in range(nq):
+            segs = np.concatenate([np.full(int(n[q]), s_ord, np.uint32) for s_ord, _, _, n in parts])
+            docs = np.concatenate([d[q, :n[q]] for _, d, _, n in parts])
+            scs = np.concatenate([sc[q, :n[q]] for _, _, sc, n in parts])
+            order = np.lexsort((docs, segs, -scs.astype(np.float64)))[top_docs.offset:top_docs.offset + k]
+            m = order.size
+            out_seg[q, :m], out_doc[q, :m], out_sc[q, :m], out_n[q] = segs[order], docs[order], scs[order], m
+        return out_seg, out_doc, out_sc, out_n
+
+    def search_phrase_batch(self, top_docs, queries_per_segment):
+        """queries_per_segment[s] is a list of PhraseQuery in segment s's own ordinals (NO_TERM where the segment does not hold
+        the term), the same phrases in the same order for every segment.  The weight of a phrase is Bm25Weight::for_terms over
+        the index-wide statistics (doc_freq summed over the segments, terms in offset order); fruits are merged as in
+        search_batch.  Returns (segment_ord [nq,k], docs [nq,k], scores [nq,k], n [nq])."""
+        nq = len(queries_per_segment[0])
+        weights = np.zeros(max(nq, 1), np.float32)
+        for q in range(nq):
+            dfs = [0] * len(queries_per_segment[0][q].term_ords)
+            for seg, qs in zip(self.segments, queries_per_segment):
+                for i, t in enumerate(qs[q].term_ords):
+                    dfs[i] += int(seg.doc_freq[t]) if t != NO_TERM else 0
+            weights[q] = Bm25Weight.for_terms(dfs, self.total_num_docs, self.average_fieldnorm).weight
+        inner = TopDocs(top_docs.limit + top_docs.offset)
+        parts = []
+        for s_ord, (seg, qs) in enumerate(zip(self.segments, queries_per_segment)):
+            d, sc, n = inner.search_phrase_batch(seg, qs, weights=weights[:nq], average_fieldnorm=self.average_fieldnorm)
             parts.append((s_ord, d, sc, n))
         k = top_docs.limit
         out_seg = np.zeros((nq, k), np.uint32); out_doc = np.zeros((nq, k), np.uint32)

@@ -77,6 +77,16 @@ struct sb200_segment {
   // sparse result tables go to the host packed (copy_out_tables)
   sb200::DevBuf<uint32_t> p_docs, p_scores; sb200::DevBuf<uint64_t> p_off;
   uint32_t* h_pack = nullptr; size_t h_pack_words = 0;   // page-locked staging: [n counts | offsets (u64) | docs | scores]
+  // positions (sb200_segment_attach_positions, bm25_phrase.cuh)
+  bool has_positions = false;
+  sb200::DevBuf<uint8_t> pos_file, pb_bits;
+  sb200::DevBuf<uint64_t> b_pos, pt_total, pt_afirst, pt_tail, pb_off;
+  sb200::DevBuf<uint32_t> pt_nb, ptail;
+  sb200::DevBuf<uint4> pa;
+  // scratch of the phrase path
+  sb200::DevBuf<uint32_t> ph_plan, ph_cq, ph_cdoc, ph_cord;
+  sb200::DevBuf<float> ph_w;
+  sb200::DevBuf<unsigned long long> ph_n;
 };
 
 namespace sb200 {
@@ -654,6 +664,7 @@ static int launch_topk_warp(const WParams& P, cudaStream_t s) {
 #include "bm25_or3.cuh"
 #include "bm25_multi.cuh"
 #include "bm25_wand.cuh"
+#include "bm25_phrase.cuh"
 namespace sb200 {
 
 static void seg_view(const sb200_segment* g, SegView& S) {
@@ -1171,6 +1182,152 @@ static int run_batch(sb200_segment* g, const sb200_bm25_batch* b, int mode, cons
   return SB200_OK;
 }
 
+
+// Phrase batch (bm25_phrase.cuh).  Host planning per query: absent term -> no scorer (phrase_weight.rs:53-62), the distinct
+// terms sorted by doc_freq (stable) with the phrase slots pointing at them, shifts = max_offset - offset.  Candidate memory is
+// sum(doc_freq of the rarest term) x (8 + 4 MAXT) B for the list + 8 B for the scored matches; slots are processed in groups
+// that keep it under a budget.
+static int run_phrase(sb200_segment* g, const sb200_phrase_batch* b, uint32_t* docs, float* scores, uint32_t* n_out, sb200_bm25_stats* stats) {
+  NvtxRange nvtx("sb200 phrase top-k batch");
+  cudaStream_t s = g->stream;
+  if (!b || !b->term_ords || !b->offsets || !b->lens || !b->weights || !b->tf_cache256 || !docs || !scores || !n_out) SB_FAIL(SB200_EINVAL, "NULL argument");
+  if (!g->has_positions) SB_FAIL(SB200_EINVAL, "the segment has no positions attached (PhraseQuery needs WithFreqsAndPositions, phrase_query.rs:106-118)");
+  const uint32_t nq = b->n_queries, nt = b->n_terms, k = b->k;
+  if (nt < 2 || nt > MAXT) SB_FAIL(SB200_ERANGE, "n_terms %u outside [2,%d]", nt, MAXT);
+  if (k == 0 || k > SB200_MAX_K) SB_FAIL(SB200_ERANGE, "k %u outside [1,%d]", k, SB200_MAX_K);
+  for (uint32_t q = 0; q < nq; q++) {
+    if (b->lens[q] < 2 || b->lens[q] > nt) SB_FAIL(SB200_EINVAL, "query %u: phrase length %u outside [2,%u] (phrase_query.rs:49-52)", q, b->lens[q], nt);
+    for (uint32_t i = 0; i < b->lens[q]; i++) {
+      const uint32_t ord = b->term_ords[(size_t)q * nt + i];
+      if (ord != SB200_NO_TERM && ord >= g->n_terms) SB_FAIL(SB200_EINVAL, "query %u: term ordinal %u >= %u", q, ord, g->n_terms);
+    }
+  }
+  // plan, one slot per query that can match: [terms | nd | len | slot | shift] as u32
+  std::vector<uint32_t> order, pterms, pnd, plen, pslot, pshift;
+  std::vector<float> pw;
+  unsigned long long postings = 0;
+  for (uint32_t q = 0; q < nq; q++) {
+    const uint32_t L = b->lens[q];
+    const uint32_t* row = b->term_ords + (size_t)q * nt;
+    bool absent = false;
+    for (uint32_t i = 0; i < L; i++) { if (row[i] == SB200_NO_TERM) absent = true; else postings += g->h_df[row[i]]; }
+    if (absent) continue;
+    uint32_t dist[MAXT], nd = 0, slot[MAXT], maxo = 0;
+    for (uint32_t i = 0; i < L; i++) {
+      uint32_t x = 0; while (x < nd && dist[x] != row[i]) x++;
+      if (x == nd) dist[nd++] = row[i];
+      maxo = std::max(maxo, b->offsets[(size_t)q * nt + i]);
+    }
+    uint32_t rank[MAXT];
+    for (uint32_t x = 0; x < nd; x++) rank[x] = x;
+    std::stable_sort(rank, rank + nd, [&](uint32_t a, uint32_t c) { return g->h_df[dist[a]] < g->h_df[dist[c]]; });
+    uint32_t where[MAXT];
+    for (uint32_t x = 0; x < nd; x++) where[rank[x]] = x;
+    for (uint32_t i = 0; i < L; i++) { uint32_t x = 0; while (dist[x] != row[i]) x++; slot[i] = where[x]; }
+    order.push_back(q);
+    for (uint32_t x = 0; x < MAXT; x++) pterms.push_back(x < nd ? dist[rank[x]] : 0u);
+    pnd.push_back(nd); plen.push_back(L); pw.push_back(b->weights[q]);
+    for (uint32_t i = 0; i < MAXT; i++) { pslot.push_back(i < L ? slot[i] : 0u); pshift.push_back(i < L ? maxo - b->offsets[(size_t)q * nt + i] : 0u); }
+  }
+  if (nq == 0) return SB200_OK;
+  const uint32_t ns = (uint32_t)order.size();
+  SB_TRY(ensure(g->o_docs, std::max<size_t>((size_t)nq * k, 1))); SB_TRY(ensure(g->o_scores, std::max<size_t>((size_t)nq * k, 1)));
+  SB_TRY(ensure(g->o_n, std::max<uint32_t>(nq, 1))); SB_TRY(ensure(g->counters, 4)); SB_TRY(ensure(g->q_cache, 256));
+  SB_TRY(ensure(g->q_orig, std::max<uint32_t>(ns, 1))); SB_TRY(ensure(g->ph_w, std::max<size_t>((size_t)ns * (MAXT + 1), 1)));
+  SB_TRY(ensure(g->ph_plan, std::max<size_t>((size_t)ns * (3 * MAXT + 2), 1))); SB_TRY(ensure(g->ph_n, 1));
+  SB_TRY(ensure(g->a3_off, std::max<uint32_t>(ns, 1))); SB_TRY(ensure(g->a3_cnt, std::max<uint32_t>(ns, 1)));
+  uint32_t* d_terms = g->ph_plan.p; uint32_t* d_slot = d_terms + (size_t)ns * MAXT; uint32_t* d_shift = d_slot + (size_t)ns * MAXT;
+  uint32_t* d_nd = d_shift + (size_t)ns * MAXT; uint32_t* d_len = d_nd + ns;
+  SB_CUDA(cudaEventRecord(g->ev0, s));
+  SB_CUDA(cudaMemsetAsync(g->o_n.p, 0, (size_t)std::max<uint32_t>(nq, 1) * 4, s));
+  SB_CUDA(cudaMemsetAsync(g->counters.p, 0, 4 * sizeof(unsigned long long), s));
+  SB_CUDA(cudaMemcpyAsync(g->q_cache.p, b->tf_cache256, 256 * 4, cudaMemcpyDefault, s));
+  if (ns) {
+    SB_CUDA(cudaMemcpyAsync(g->q_orig.p, order.data(), (size_t)ns * 4, cudaMemcpyHostToDevice, s));
+    SB_CUDA(cudaMemcpyAsync(d_terms, pterms.data(), pterms.size() * 4, cudaMemcpyHostToDevice, s));
+    SB_CUDA(cudaMemcpyAsync(d_slot, pslot.data(), pslot.size() * 4, cudaMemcpyHostToDevice, s));
+    SB_CUDA(cudaMemcpyAsync(d_shift, pshift.data(), pshift.size() * 4, cudaMemcpyHostToDevice, s));
+    SB_CUDA(cudaMemcpyAsync(d_nd, pnd.data(), pnd.size() * 4, cudaMemcpyHostToDevice, s));
+    SB_CUDA(cudaMemcpyAsync(d_len, plen.data(), plen.size() * 4, cudaMemcpyHostToDevice, s));
+    SB_CUDA(cudaMemcpyAsync(g->ph_w.p, pw.data(), pw.size() * 4, cudaMemcpyHostToDevice, s));
+    SB_CUDA(cudaMemsetAsync(g->ph_w.p + ns, 0, (size_t)ns * MAXT * 4, s));
+  }
+  static size_t sel_conf = 0;
+  const size_t sel_smem = (size_t)A3_SEL_CAP * 8;
+  if (sel_conf < sel_smem) {
+    SB_CUDA(cudaFuncSetAttribute(k_and3_select, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sel_smem));
+    sel_conf = sel_smem;
+  }
+  const uint64_t max_entries = std::max<uint64_t>(((uint64_t)4 << 30) / (16 + 4 * MAXT), 1);
+  std::vector<uint64_t> off(std::max<uint32_t>(ns, 1), 0);
+  std::vector<AUnit> units;
+  unsigned long long n_cand = 0;
+  SB_CUDA(cudaEventRecord(g->evk0, s));
+  uint32_t g0 = 0;
+  while (g0 < ns) {
+    uint64_t entries = 0; uint32_t g1 = g0;
+    units.clear();
+    while (g1 < ns) {
+      const uint32_t dfA = g->h_df[pterms[(size_t)g1 * MAXT]];
+      if (g1 > g0 && entries + dfA > max_entries) break;
+      off[g1] = entries; entries += dfA;
+      const uint32_t nblk = (dfA >> 7) + ((dfA & 127u) ? 1u : 0u);
+      for (uint32_t b0 = 0; b0 < nblk; b0 += A3_UNIT_BLOCKS) {
+        AUnit u; u.q = g1; u.blk_lo = b0; u.blk_hi = std::min(nblk, b0 + A3_UNIT_BLOCKS); u._pad = 0;
+        units.push_back(u);
+      }
+      g1++;
+    }
+    const uint32_t n_units = (uint32_t)units.size();
+    const size_t cap = (size_t)std::max<uint64_t>(entries, 1);
+    SB_TRY(ensure(g->ph_cq, cap)); SB_TRY(ensure(g->ph_cdoc, cap)); SB_TRY(ensure(g->ph_cord, cap * MAXT));
+    SB_TRY(ensure(g->a3_key, cap)); SB_TRY(ensure(g->a3_doc, cap)); SB_TRY(ensure(g->a3_units, std::max<size_t>(n_units, 1)));
+    SB_CUDA(cudaMemcpyAsync(g->a3_off.p + g0, off.data() + g0, (size_t)(g1 - g0) * 8, cudaMemcpyHostToDevice, s));
+    SB_CUDA(cudaMemsetAsync(g->a3_cnt.p + g0, 0, (size_t)(g1 - g0) * 4, s));
+    SB_CUDA(cudaMemsetAsync(g->ph_n.p, 0, sizeof(unsigned long long), s));
+    if (n_units) {
+      SB_CUDA(cudaMemcpyAsync(g->a3_units.p, units.data(), (size_t)n_units * sizeof(AUnit), cudaMemcpyHostToDevice, s));
+      PhParams PP;
+      memset(&PP, 0, sizeof(PP));
+      A3Params& A = PP.A;
+      seg_view(g, A.S); A.a128 = g->a_post.p; A.t_aoff = g->t_aoff.p;
+      A.q_terms = d_terms; A.q_nterms = d_nd; A.q_weights = g->ph_w.p + ns; A.cache = g->q_cache.p; A.n_terms_max = MAXT;
+      A.units = (const AUnit*)g->a3_units.p; A.n_units = n_units; A.counters = g->counters.p;
+      PP.b_pos = g->b_pos.p; PP.pa = g->pa.p; PP.pb_off = g->pb_off.p; PP.pb_bits = g->pb_bits.p;
+      PP.pt_afirst = g->pt_afirst.p; PP.pt_nb = g->pt_nb.p; PP.pt_tail = g->pt_tail.p; PP.ptail = g->ptail.p; PP.pt_total = g->pt_total.p;
+      PP.q_len = d_len; PP.q_slot = d_slot; PP.q_shift = d_shift; PP.q_weight = g->ph_w.p;
+      PP.c_q = g->ph_cq.p; PP.c_doc = g->ph_cdoc.p; PP.c_ord = g->ph_cord.p; PP.c_n = g->ph_n.p; PP.c_cap = cap;
+      PP.r_off = g->a3_off.p; PP.r_cnt = g->a3_cnt.p; PP.r_key = g->a3_key.p; PP.r_doc = g->a3_doc.p; PP.counters = g->counters.p;
+      SB_LAUNCH(k_phrase_docs, div_up(n_units, A3_WARPS), A3_WARPS * 32, 0, s, PP);
+      SB_CHECK_LAUNCH();
+      const unsigned grid = (unsigned)std::min<uint64_t>(div_up(cap, A3_WARPS), 148u * 16u);
+      SB_LAUNCH(k_phrase_match, grid, A3_WARPS * 32, 0, s, PP);
+      SB_CHECK_LAUNCH();
+    }
+    SB_LAUNCH(k_and3_select, g1 - g0, 256, sel_smem, s, g->a3_off.p, g->a3_cnt.p, g->a3_key.p, g->a3_doc.p, g->q_orig.p, g0, k,
+              g->o_docs.p, g->o_scores.p, g->o_n.p);
+    SB_CHECK_LAUNCH();
+    unsigned long long c = 0;
+    SB_CUDA(cudaMemcpyAsync(&c, g->ph_n.p, sizeof(c), cudaMemcpyDeviceToHost, s));
+    SB_CUDA(cudaStreamSynchronize(s));   // `units` / `off` are reused by the next group's async copies
+    n_cand += c;
+    g0 = g1;
+  }
+  SB_CUDA(cudaEventRecord(g->evk1, s));
+  SB_TRY(copy_out_tables(g, nq, k, docs, scores, nullptr, n_out));
+  unsigned long long h[4] = {0, 0, 0, 0};
+  SB_CUDA(cudaMemcpyAsync(h, g->counters.p, sizeof(h), cudaMemcpyDeviceToHost, s));
+  SB_CUDA(cudaEventRecord(g->ev1, s));
+  SB_CUDA(cudaStreamSynchronize(s));
+  if (h[2]) SB_FAIL(SB200_EFORMAT, "%llu phrase work items met inconsistent posting or position data", h[2]);
+  if (stats) {
+    float ms = 0; cudaEventElapsedTime(&ms, g->ev0, g->ev1);
+    stats->postings_scored = postings; stats->docs_scored = n_cand; stats->blocks_decoded = h[1]; stats->ms = ms;
+    cudaEventElapsedTime(&stats->kernel_ms, g->evk0, g->evk1);
+  }
+  return SB200_OK;
+}
+
 }  // namespace sb200
 using namespace sb200;
 
@@ -1190,7 +1347,7 @@ __device__ __forceinline__ uint64_t tis_bits(const uint8_t* data, uint64_t len, 
   return v & ((1ull << nb) - 1ull);
 }
 __global__ void k_term_info_store(const uint8_t* __restrict__ file, uint64_t len, uint64_t meta_len, uint64_t n_terms,
-                                  sb200_term_info* out, int* err) {
+                                  sb200_term_info* out, uint64_t* pos_s, uint64_t* pos_e, int* err) {
   const uint64_t ord = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
   if (ord >= n_terms) return;
   const uint8_t* m = file + 16 + (ord >> 8) * 47;
@@ -1202,8 +1359,10 @@ __global__ void k_term_info_store(const uint8_t* __restrict__ file, uint64_t len
   const uint32_t dfb = m[44], pb = m[45], qb = m[46];
   const uint32_t inner = (uint32_t)(ord & 255u);
   sb200_term_info ti; ti._pad = 0;
-  if (inner == 0) { ti.postings_off = rps; ti.postings_len = rpl; ti.doc_freq = rdf; }
-  else {
+  if (inner == 0) {
+    ti.postings_off = rps; ti.postings_len = rpl; ti.doc_freq = rdf;
+    if (pos_s) { const uint64_t qs = tis_u64(m + 28, 8); pos_s[ord] = qs; pos_e[ord] = qs + tis_u64(m + 36, 8); }
+  } else {
     if (off > infos_len || dfb > 56 || pb > 56 || qb > 56) { *err = 1; return; }
     const uint64_t nb = (uint64_t)dfb + pb + qb, a0 = nb * (inner - 1);
     const uint8_t* d = infos + off; const uint64_t dl = infos_len - off;
@@ -1211,6 +1370,12 @@ __global__ void k_term_info_store(const uint8_t* __restrict__ file, uint64_t len
     if (pe < ps) { *err = 2; return; }
     ti.postings_off = ps; ti.postings_len = pe - ps;
     ti.doc_freq = (uint32_t)tis_bits(d, dl, a0 + pb + qb, dfb);
+    if (pos_s) {   // positions_range: start at a0 + pb, end = the next term's start (term_info_store.rs:66-91)
+      const uint64_t qs = tis_u64(m + 28, 8);
+      const uint64_t s0 = qs + tis_bits(d, dl, a0 + pb, qb), s1 = qs + tis_bits(d, dl, a0 + pb + nb, qb);
+      if (s1 < s0) { *err = 3; return; }
+      pos_s[ord] = s0; pos_e[ord] = s1;
+    }
   }
   out[ord] = ti;
 }
@@ -1218,8 +1383,8 @@ __global__ void k_term_info_store(const uint8_t* __restrict__ file, uint64_t len
 
 extern "C" {
 
-int sb200_term_info_store_decode(const uint8_t* store, uint64_t len, int device, sb200_term_info* infos, uint64_t cap,
-                                 uint64_t* n_terms) {
+static int tis_decode(const uint8_t* store, uint64_t len, int device, sb200_term_info* infos, uint64_t* pos_start, uint64_t* pos_end,
+                      uint64_t cap, uint64_t* n_terms) {
   using namespace sb200;
   if (!store || !n_terms) SB_FAIL(SB200_EINVAL, "NULL argument");
   if (len < 16) SB_FAIL(SB200_EFORMAT, "term info store shorter than its 16-byte header");
@@ -1231,18 +1396,35 @@ int sb200_term_info_store_decode(const uint8_t* store, uint64_t len, int device,
   if (meta_len > len - 16 || meta_len != 47ull * ((n + 255) / 256)) SB_FAIL(SB200_EFORMAT, "term info store: %llu terms need %llu bytes of block metadata, header says %llu", (unsigned long long)n, (unsigned long long)(47ull * ((n + 255) / 256)), (unsigned long long)meta_len);
   *n_terms = n;
   const uint64_t k = std::min<uint64_t>(n, cap);
-  if (!infos || k == 0) return SB200_OK;
-  DevBuf<uint8_t> d_store; DevBuf<sb200_term_info> d_out; DevBuf<int> d_err;
+  if ((!infos && !pos_start) || k == 0) return SB200_OK;
+  DevBuf<uint8_t> d_store; DevBuf<sb200_term_info> d_out; DevBuf<int> d_err; DevBuf<uint64_t> d_pos;
   SB_TRY(d_store.alloc(len)); SB_TRY(d_out.alloc(n)); SB_TRY(d_err.alloc(1));
+  if (pos_start) SB_TRY(d_pos.alloc(2 * n));
   SB_CUDA(cudaMemcpy(d_store.p, store, len, cudaMemcpyDefault));
   SB_CUDA(cudaMemset(d_err.p, 0, sizeof(int)));
-  SB_LAUNCH(k_term_info_store, div_up(n, 256), 256, 0, (cudaStream_t)0, d_store.p, len, meta_len, n, d_out.p, d_err.p);
+  SB_LAUNCH(k_term_info_store, div_up(n, 256), 256, 0, (cudaStream_t)0, d_store.p, len, meta_len, n, d_out.p,
+            pos_start ? d_pos.p : nullptr, pos_start ? d_pos.p + n : nullptr, d_err.p);
   SB_CHECK_LAUNCH();
   int h_err = 0;
   SB_CUDA(cudaMemcpy(&h_err, d_err.p, sizeof(int), cudaMemcpyDeviceToHost));
   if (h_err) SB_FAIL(SB200_EFORMAT, "term info store is inconsistent (code %d)", h_err);
-  SB_CUDA(cudaMemcpy(infos, d_out.p, k * sizeof(sb200_term_info), cudaMemcpyDefault));
+  if (infos) SB_CUDA(cudaMemcpy(infos, d_out.p, k * sizeof(sb200_term_info), cudaMemcpyDefault));
+  if (pos_start) {
+    SB_CUDA(cudaMemcpy(pos_start, d_pos.p, k * 8, cudaMemcpyDefault));
+    SB_CUDA(cudaMemcpy(pos_end, d_pos.p + n, k * 8, cudaMemcpyDefault));
+  }
   return SB200_OK;
+}
+
+int sb200_term_info_store_decode(const uint8_t* store, uint64_t len, int device, sb200_term_info* infos, uint64_t cap,
+                                 uint64_t* n_terms) {
+  return tis_decode(store, len, device, infos, nullptr, nullptr, cap, n_terms);
+}
+
+int sb200_term_info_store_decode_positions(const uint8_t* store, uint64_t len, int device, uint64_t* pos_start, uint64_t* pos_end,
+                                           uint64_t cap, uint64_t* n_terms) {
+  if (cap && (!pos_start || !pos_end)) SB_FAIL(SB200_EINVAL, "NULL argument");
+  return tis_decode(store, len, device, nullptr, cap ? pos_start : nullptr, pos_end, cap, n_terms);
 }
 
 int sb200_segment_create(const uint8_t* postings_file, uint64_t postings_len, const sb200_term_info* terms, uint32_t n_terms,
@@ -1352,7 +1534,9 @@ int sb200_segment_get_info(const sb200_segment* g, sb200_segment_info* info) {
   if (!g || !info) SB_FAIL(SB200_EINVAL, "NULL argument");
   info->n_terms = g->n_terms; info->n_blocks = g->n_blocks; info->n_postings = g->n_postings; info->max_doc = g->max_doc; info->_pad = 0;
   info->hbm_bytes = g->postings.bytes() + g->fieldnorm.bytes() + g->t_first.bytes() + g->t_data_off.bytes() + g->t_end_off.bytes() +
-                    g->t_df.bytes() + g->b_last.bytes() + g->b_off.bytes() + g->b_bits.bytes() + g->b_bw.bytes();
+                    g->t_df.bytes() + g->b_last.bytes() + g->b_off.bytes() + g->b_bits.bytes() + g->b_bw.bytes() +
+                    g->pos_file.bytes() + g->pb_bits.bytes() + g->b_pos.bytes() + g->pt_total.bytes() + g->pt_afirst.bytes() +
+                    g->pt_tail.bytes() + g->pb_off.bytes() + g->pt_nb.bytes() + g->ptail.bytes() + g->pa.bytes();
   info->stage_ms = g->stage_ms;
   return SB200_OK;
 }
@@ -1462,6 +1646,83 @@ void sb200_signals_destroy(sb200_signals* s) {
   if (!s) return;
   cudaSetDevice(s->device);
   delete s;
+}
+
+int sb200_segment_attach_positions(sb200_segment* g, const uint8_t* positions_file, uint64_t len, const uint64_t* pos_start,
+                                   const uint64_t* pos_end) {
+  if (!g) SB_FAIL(SB200_EINVAL, "NULL segment handle");
+  if (g->record != SB200_RECORD_FREQS_POSITIONS) SB_FAIL(SB200_EINVAL, "positions need a WithFreqsAndPositions segment (record option 2), this one has %d", g->record);
+  if ((len && !positions_file) || (g->n_terms && (!pos_start || !pos_end))) SB_FAIL(SB200_EINVAL, "NULL argument");
+  SB_CUDA(cudaSetDevice(g->device));
+  const uint32_t nt = g->n_terms;
+  std::vector<uint64_t> hs(nt), he(nt);
+  if (nt) {
+    SB_CUDA(cudaMemcpy(hs.data(), pos_start, (size_t)nt * 8, cudaMemcpyDefault));
+    SB_CUDA(cudaMemcpy(he.data(), pos_end, (size_t)nt * 8, cudaMemcpyDefault));
+  }
+  for (uint32_t t = 0; t < nt; t++)
+    if (hs[t] > he[t] || he[t] > len) SB_FAIL(SB200_EFORMAT, "term %u: positions range [%llu, %llu) outside the %llu-byte file", t,
+                                              (unsigned long long)hs[t], (unsigned long long)he[t], (unsigned long long)len);
+  g->has_positions = false;
+  cudaStream_t s = g->stream;
+  auto body = [&]() -> int {
+    SB_TRY(g->pos_file.alloc(len + 64));
+    SB_CUDA(cudaMemsetAsync(g->pos_file.p + len, 0, 64, s));
+    if (len) SB_TRY(copy_in(g->pos_file.p, positions_file, len, s));
+    const size_t slots = g->b_last.n;
+    SB_TRY(g->b_pos.alloc(slots)); SB_TRY(g->pt_total.alloc(nt + 1)); SB_TRY(g->pt_nb.alloc(nt + 1));
+    DevBuf<uint64_t> d_se, d_hdr, d_packed, d_au; DevBuf<int> d_err;
+    SB_TRY(d_se.alloc(2 * (size_t)nt + 2)); SB_TRY(d_hdr.alloc(nt + 1)); SB_TRY(d_packed.alloc(nt + 1)); SB_TRY(d_err.alloc(1));
+    SB_CUDA(cudaMemcpyAsync(d_se.p, hs.data(), (size_t)nt * 8, cudaMemcpyHostToDevice, s));
+    SB_CUDA(cudaMemcpyAsync(d_se.p + nt, he.data(), (size_t)nt * 8, cudaMemcpyHostToDevice, s));
+    SB_CUDA(cudaMemsetAsync(d_err.p, 0, sizeof(int), s));
+    if (nt) {
+      SB_LAUNCH(k_pos_scan, div_up((uint64_t)nt * 32, 256), 256, 0, s, g->postings.p, g->t_first.p, g->t_df.p, g->t_data_off.p, g->t_end_off.p,
+                g->b_off.p, nt, g->pos_file.p, d_se.p, d_se.p + nt, g->b_pos.p, g->pt_total.p, g->pt_nb.p, d_hdr.p, d_packed.p, d_err.p);
+      SB_CHECK_LAUNCH();
+    }
+    int h_err = 0;
+    SB_CUDA(cudaMemcpyAsync(&h_err, d_err.p, sizeof(int), cudaMemcpyDeviceToHost, s));
+    std::vector<uint64_t> total(nt), packed(nt); std::vector<uint32_t> nb(nt);
+    if (nt) {
+      SB_CUDA(cudaMemcpyAsync(total.data(), g->pt_total.p, (size_t)nt * 8, cudaMemcpyDeviceToHost, s));
+      SB_CUDA(cudaMemcpyAsync(packed.data(), d_packed.p, (size_t)nt * 8, cudaMemcpyDeviceToHost, s));
+      SB_CUDA(cudaMemcpyAsync(nb.data(), g->pt_nb.p, (size_t)nt * 4, cudaMemcpyDeviceToHost, s));
+    }
+    SB_CUDA(cudaStreamSynchronize(s));
+    if (h_err) SB_FAIL(SB200_EFORMAT, "malformed positions (code %d): bad block count or vint, block count != term frequency sum / 128, "
+                                      "bit width > 32, blocks past the term's range, or a tail that is not term frequency sum %% 128 vints", h_err);
+    std::vector<uint64_t> afirst(nt + 1), aunits(nt + 1), tail(nt + 1);
+    uint64_t a = 0, u = 0, tl = 0;
+    for (uint32_t t = 0; t < nt; t++) { afirst[t] = a; aunits[t] = u; tail[t] = tl; a += nb[t]; u += packed[t] >> 4; tl += total[t] & 127u; }
+    SB_TRY(g->pt_afirst.alloc(nt + 1)); SB_TRY(g->pt_tail.alloc(nt + 1)); SB_TRY(d_au.alloc(nt + 1));
+    SB_TRY(g->pb_off.alloc(a + 1)); SB_TRY(g->pb_bits.alloc(a + 1)); SB_TRY(g->pa.alloc(u + 1)); SB_TRY(g->ptail.alloc(tl + 1));
+    if (nt) {
+      SB_CUDA(cudaMemcpyAsync(g->pt_afirst.p, afirst.data(), (size_t)nt * 8, cudaMemcpyHostToDevice, s));
+      SB_CUDA(cudaMemcpyAsync(g->pt_tail.p, tail.data(), (size_t)nt * 8, cudaMemcpyHostToDevice, s));
+      SB_CUDA(cudaMemcpyAsync(d_au.p, aunits.data(), (size_t)nt * 8, cudaMemcpyHostToDevice, s));
+      SB_LAUNCH(k_pos_build, div_up((uint64_t)nt * 32, 256), 256, 0, s, g->pos_file.p, nt, d_hdr.p, g->pt_nb.p, d_packed.p, g->pt_total.p,
+                g->pt_afirst.p, d_au.p, g->pt_tail.p, g->pb_off.p, g->pb_bits.p, (uint32_t*)g->pa.p, g->ptail.p);
+      SB_CHECK_LAUNCH();
+    }
+    SB_CUDA(cudaStreamSynchronize(s));
+    return SB200_OK;
+  };
+  const int rc = body();
+  if (rc != SB200_OK) {
+    g->pos_file.release(); g->pb_bits.release(); g->b_pos.release(); g->pt_total.release(); g->pt_afirst.release(); g->pt_tail.release();
+    g->pb_off.release(); g->pt_nb.release(); g->ptail.release(); g->pa.release();
+    return rc;
+  }
+  g->has_positions = true;
+  return SB200_OK;
+}
+
+int sb200_phrase_topk_batch(sb200_segment* seg, const sb200_phrase_batch* batch, uint32_t* docs, float* scores, uint32_t* n_out,
+                            sb200_bm25_stats* stats) {
+  if (!seg) SB_FAIL(SB200_EINVAL, "NULL segment handle");
+  SB_CUDA(cudaSetDevice(seg->device));
+  return run_phrase(seg, batch, docs, scores, n_out, stats);
 }
 
 int sb200_bm25_topk_batch(sb200_segment* seg, const sb200_bm25_batch* batch, uint32_t* docs, float* scores, uint32_t* n_out,

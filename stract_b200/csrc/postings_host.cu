@@ -111,6 +111,39 @@ void encode_term(const uint32_t* docs, const uint32_t* tfs, uint32_t df, const u
   out.insert(out.end(), body.begin(), body.end());
 }
 
+// PositionSerializer::write_positions_delta + close_term for one term (tantivy/src/positions/serializer.rs, format in
+// positions/mod.rs:7-30): VInt(#full blocks), one bit width per block, the blocks (BitPacker4x, unsorted, not minus-one
+// encoded: compression/mod.rs:51-67), then the P % 128 remaining deltas as unsorted vints (compression/vint.rs:24-42).
+// `pos` holds the term's Σtf absolute positions posting by posting; a document's first delta is its first position
+// (postings/serializer.rs:191-205).  Returns false when a document's positions are not strictly ascending.
+bool encode_positions_term(const uint32_t* tfs, uint32_t df, const uint32_t* pos, std::vector<uint8_t>& out) {
+  std::vector<uint32_t> delta;
+  uint64_t n = 0;
+  for (uint32_t i = 0; i < df; i++) n += tfs[i];
+  delta.resize(n);
+  uint64_t at = 0;
+  for (uint32_t i = 0; i < df; i++) {
+    uint32_t prev = 0;
+    for (uint32_t j = 0; j < tfs[i]; j++, at++) {
+      if (j && pos[at] <= prev) return false;
+      delta[at] = pos[at] - prev; prev = pos[at];
+    }
+  }
+  const uint64_t nb = n / 128;
+  std::vector<uint8_t> widths(nb), body;
+  for (uint64_t b = 0; b < nb; b++) {
+    uint32_t orred = 0;
+    for (int i = 0; i < 128; i++) orred |= delta[b * 128 + i];
+    widths[b] = (uint8_t)width_of(orred);
+    pack4x(delta.data() + b * 128, widths[b], body);
+  }
+  for (uint64_t i = nb * 128; i < n; i++) put_vint(body, delta[i]);
+  put_vint(out, nb);
+  out.insert(out.end(), widths.begin(), widths.end());
+  out.insert(out.end(), body.begin(), body.end());
+  return true;
+}
+
 }  // namespace
 }  // namespace sb200
 
@@ -181,6 +214,56 @@ int sb200_postings_encode_ex(const uint32_t* docs, const uint32_t* tfs, const ui
     if (infos) { infos[t].postings_off = at; infos[t].postings_len = enc[t].bytes.size(); infos[t].doc_freq = (uint32_t)(term_off[t + 1] - term_off[t]); infos[t]._pad = 0; }
     memcpy(out + at, enc[t].bytes.data(), enc[t].bytes.size());
     at += enc[t].bytes.size();
+  }
+  return SB200_OK;
+}
+
+int sb200_positions_encode(const uint32_t* docs, const uint32_t* tfs, const uint64_t* term_off, uint32_t n_terms,
+                           const uint32_t* positions, uint8_t* out, uint64_t out_cap, uint64_t* out_len, uint64_t* pos_start,
+                           uint64_t* pos_end, int threads) {
+  using namespace sb200;
+  if (!term_off || !out_len || (n_terms && (!docs || !tfs || !positions))) SB_FAIL(SB200_EINVAL, "NULL argument");
+  // positions of posting i of term t start at Σ tfs[..i] over the whole CSR
+  std::vector<uint64_t> pos_off(n_terms + 1, 0);
+  for (uint32_t t = 0; t < n_terms; t++) {
+    const uint64_t a = term_off[t], b = term_off[t + 1];
+    if (b < a || b - a > 0x7FFFFFFFull) SB_FAIL(SB200_EINVAL, "term %u: term_off is not ascending", t);
+    uint64_t s = 0;
+    for (uint64_t i = a; i < b; i++) s += tfs[i];
+    pos_off[t + 1] = pos_off[t] + s;
+  }
+  std::vector<TermBytes> enc(n_terms);
+  std::atomic<uint32_t> next(0);
+  std::atomic<int> bad(0);
+  auto work = [&]() {
+    for (;;) {
+      const uint32_t t = next.fetch_add(64);
+      if (t >= n_terms) break;
+      for (uint32_t u = t; u < std::min(n_terms, t + 64); u++) {
+        const uint64_t a = term_off[u];
+        const uint32_t df = (uint32_t)(term_off[u + 1] - a);
+        for (uint32_t i = 0; i < df; i++) if (tfs[a + i] == 0 || (i && docs[a + i] <= docs[a + i - 1])) { bad = 1; break; }
+        if (!bad && !encode_positions_term(tfs + a, df, positions + pos_off[u], enc[u].bytes)) bad = 2;
+      }
+    }
+  };
+  const int nt = std::max(1, threads);
+  std::vector<std::thread> pool;
+  for (int i = 0; i < nt; i++) pool.emplace_back(work);
+  for (auto& th : pool) th.join();
+  if (bad == 1) SB_FAIL(SB200_EINVAL, "posting input must be ascending doc ids with tf >= 1");
+  if (bad == 2) SB_FAIL(SB200_EINVAL, "the positions of a document must be strictly ascending");
+  uint64_t total = 0;
+  for (uint32_t t = 0; t < n_terms; t++) total += enc[t].bytes.size();
+  *out_len = total;
+  if (!out) return SB200_OK;
+  if (out_cap < total) SB_FAIL(SB200_EINVAL, "output buffer too small: need %llu bytes", (unsigned long long)total);
+  uint64_t at = 0;
+  for (uint32_t t = 0; t < n_terms; t++) {
+    if (pos_start) pos_start[t] = at;
+    memcpy(out + at, enc[t].bytes.data(), enc[t].bytes.size());
+    at += enc[t].bytes.size();
+    if (pos_end) pos_end[t] = at;
   }
   return SB200_OK;
 }
